@@ -50,7 +50,8 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 import numpy as np  # noqa: E402
 
-CACHE = os.environ.get("WM_BENCH_CACHE", "/tmp/wm_bench_cache")
+# per user: on a shared machine another user's cache directory is not writable
+CACHE = os.environ.get("WM_BENCH_CACHE", os.path.join(tempfile.gettempdir(), f"wm_bench_cache_{os.getuid()}"))
 REF_LEN = int(os.environ.get("WM_BENCH_REF_LEN", 500_000_000))
 GROUP = max(1, int(os.environ.get("WM_BENCH_GROUP", 32)))
 N50, ERR, K = 30000, 0.05, 15
@@ -223,6 +224,62 @@ def run_reference(refbin, ref, wf, reads_fa, threads, out_path=None, mini_batch=
     return t_idx, stamps
 
 
+# wm_reg1_t (include/winnowmap_b200.h): 15 int32, the bit-field word (mapq:8 split:2 rev:1 inv:1 sam_pri:1 ...), hash, div, ->p
+REG1 = np.dtype([(f, "<i4") for f in ("id", "cnt", "rid", "score", "qs", "qe", "rs", "re", "parent", "subsc", "as", "mlen", "blen", "n_sub",
+                                      "score0")] + [("bits", "<u4"), ("hash", "<u4"), ("div", "<f4"), ("p", "<u8")])
+# reads of the last step dumped: a seeded sample of at most this many bases (all of a default step) -- about 0.45 byte of
+# output per base on the bench workload, so the files stay well under DUMP_LIMIT
+DUMP_BASES = 32_000_000
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(L, ctx, step_reads, first, out_dir):
+    """The records the timed (resident) pass returned for the reads of its last step -- a fixed sample of them, drawn from the
+    inputs alone -- as float64 arrays out_dir/<name>.npy: per read (read_*), per record (reg_*) and the CIGARs of the records,
+    concatenated (cigar, len << 4 | op; reg_n_cigar says where each record's ops end)."""
+    order = np.random.default_rng(0).permutation(len(step_reads))
+    n_keep = int(np.searchsorted(np.cumsum([len(step_reads[i][1]) for i in order]), DUMP_BASES, side="right"))
+    keep = np.sort(order[:max(1, n_keep)])
+    L.wm_sizeof_reg1.restype = C.c_int
+    assert L.wm_sizeof_reg1() == REG1.itemsize
+    L.wm_bench_records.restype = C.c_int64
+    L.wm_bench_records.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
+    out = {k: [] for k in ["read_index", "read_n_reg", "read_rep_len", "reg_read"] + [f"reg_{f}" for f in REG1.names[:15]] +
+           ["reg_mapq", "reg_split", "reg_rev", "reg_inv", "reg_sam_pri", "reg_hash", "reg_div", "reg_dp_score", "reg_dp_max",
+            "reg_dp_max2", "reg_n_ambi", "reg_trans_strand", "reg_n_cigar", "cigar"]}
+    n_reg, rep_len = np.zeros(1, np.int32), np.zeros(1, np.int32)
+    for i in keep:
+        n = L.wm_bench_records(ctx, first + int(i), 1, n_reg.ctypes.data, rep_len.ctypes.data, None, 0)
+        regs = np.zeros(n, REG1)
+        L.wm_bench_records(ctx, first + int(i), 1, n_reg.ctypes.data, rep_len.ctypes.data, regs.ctypes.data, n)
+        out["read_index"].append(i); out["read_n_reg"].append(n_reg[0]); out["read_rep_len"].append(rep_len[0])
+        for r in regs:
+            out["reg_read"].append(i)
+            for f in REG1.names[:15]:
+                out[f"reg_{f}"].append(r[f])
+            b = int(r["bits"])
+            for f, sh, w in (("mapq", 0, 8), ("split", 8, 2), ("rev", 10, 1), ("inv", 11, 1), ("sam_pri", 12, 1)):
+                out[f"reg_{f}"].append((b >> sh) & ((1 << w) - 1))
+            out["reg_hash"].append(r["hash"]); out["reg_div"].append(r["div"])
+            # wm_extra_t: capacity, dp_score, dp_max, dp_max2, n_ambi:30 | trans_strand:2, n_cigar, cigar[]
+            ex = np.frombuffer(C.string_at(int(r["p"]), 24), np.int32) if r["p"] else np.zeros(6, np.int32)
+            for f, v in zip(("dp_score", "dp_max", "dp_max2"), ex[1:4]):
+                out[f"reg_{f}"].append(v)
+            amb = int(ex[4]) & 0xffffffff
+            out["reg_n_ambi"].append(amb & 0x3fffffff); out["reg_trans_strand"].append(amb >> 30); out["reg_n_cigar"].append(ex[5])
+            if ex[5] > 0:
+                out["cigar"].append(np.frombuffer(C.string_at(int(r["p"]) + 24, 4 * int(ex[5])), np.uint32))
+    out["cigar"] = np.concatenate(out["cigar"]) if out["cigar"] else np.zeros(0)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in out.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT}")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    log(f"dumped {len(keep)} of {len(step_reads)} reads of the last step, {len(arrays['reg_read'])} records, {total / 1e6:.1f} MB to {out_dir}")
+
+
 def paf_by_read(path):
     """read name -> list of its lines, in file order (the reference prints a mini-batch sorted by length, we print in input order)."""
     d = {}
@@ -282,6 +339,7 @@ def main():
     ap.add_argument("--cpu-reads", type=int, default=int(os.environ.get("WM_BENCH_CPU_READS", 8000)), help="reads of the cpu_baseline / parity sample")
     ap.add_argument("--cpu-reads-per-step", type=int, default=int(os.environ.get("WM_BENCH_CPU_READS_PER_STEP", 500)),
                     help="--impl reference: reads per step (a bounded sample of the step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the timed pass's last step to DIR/<name>.npy (float64)")
     a = ap.parse_args()
     rank = int(os.environ.get("RANK", 0)); world = int(os.environ.get("WORLD_SIZE", 1)); local = int(os.environ.get("LOCAL_RANK", 0))
     cores = os.cpu_count() or 1
@@ -452,6 +510,8 @@ def main():
         dist.destroy_process_group()
     if rank != 0:
         return
+    if a.dump_outputs:
+        dump_outputs(L, mp.ctx, timed[len(timed) - a.reads:], len(timed) - a.reads, a.dump_outputs)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))

@@ -290,6 +290,9 @@ int wm_format_batch(const wm_gpu_ctx *ctx, const wm_mapopt_t *opt, int n_seq, co
 int wm_bench_upload(wm_gpu_ctx *ctx, int n_seq, const char *const *names, const char *const *seqs, const int32_t *lens);
 int wm_bench_map_resident(wm_gpu_ctx *ctx, const wm_mapopt_t *opt, int n_threads, int group_reads, double *ms);
 int wm_bench_write(wm_gpu_ctx *ctx, const wm_mapopt_t *opt, int n_first, const char *out_fn);
+/* bench: n_reg[i] and rep_len[i] of reads first .. first + n - 1 of the last resident pass, and their records in input order into
+ * regs (at most cap of them; each ->p stays owned by the context until the next pass).  Returns the number of records. */
+int64_t wm_bench_records(const wm_gpu_ctx *ctx, int first, int n, int32_t *n_reg, int32_t *rep_len, wm_reg1_t *regs, int64_t cap);
 
 /* bench instrumentation (csrc/prof.cu): launch counter and CUDA-event timing of the two dominant kernel classes */
 void wm_prof_enable(int on);

@@ -1,6 +1,9 @@
 """ctypes bindings for the CPU oracle (oracle/libwm_oracle.so, a restatement) and for the
-real reference (oracle/_ref/libref_harness.so).  TEST INFRASTRUCTURE ONLY."""
+real reference (oracle/_ref/libref_harness.so), and the recorded answers of the reference
+(RefGolden) that the tests compare with where the reference is not built.  TEST INFRASTRUCTURE ONLY."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -8,6 +11,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
+REF_GOLDEN_DIR = os.path.join(ROOT, "tests", "golden", "ref")
+# WM_RECORD_REF_GOLDEN=1 (with oracle/_ref built): the tests call the reference and rewrite tests/golden/ref/
+RECORD = os.environ.get("WM_RECORD_REF_GOLDEN") == "1"
 _u8p = C.POINTER(C.c_uint8)
 _i8p = C.POINTER(C.c_int8)
 _u32p = C.POINTER(C.c_uint32)
@@ -69,6 +75,68 @@ def oracle():
 
 def have_ref():
     return os.path.exists(os.path.join(ORACLE_DIR, "_ref", "libref_harness.so"))
+
+
+def _feed(h, v):
+    if isinstance(v, np.ndarray):
+        h.update(f"a{v.dtype.str}{v.shape}".encode())
+        h.update(np.ascontiguousarray(v).tobytes())
+    elif isinstance(v, (tuple, list)):
+        h.update(b"(%d" % len(v))
+        for x in v:
+            _feed(h, x)
+        h.update(b")")
+    elif isinstance(v, bytes):
+        h.update(b"b%d:" % len(v) + v)
+    else:
+        h.update(repr(v.item() if isinstance(v, np.generic) else v).encode())
+
+
+def digest(v):
+    """64-bit fingerprint of a result (arrays with dtype and shape, ints, bools, bytes, nested tuples / lists)."""
+    h = hashlib.sha256()
+    _feed(h, v)
+    return h.hexdigest()[:16]
+
+
+class RefGolden:
+    """What the reference returned for the calls of one test, recorded in call order as digests of the results in
+    tests/golden/ref/<module>.json (the results themselves -- sorted arrays, sketches, CIGARs -- are too large to store).
+
+    check(ref_fn, got) compares `got` with the reference's answer: the recorded one, or -- with WM_RECORD_REF_GOLDEN=1
+    and oracle/_ref built from the reference -- ref_fn(), whose digest is then recorded (the file is written after
+    every call).  ref_fn is not called otherwise, so it may use objects that only exist when recording."""
+    _files = {}
+
+    def __init__(self, request):
+        self.path = os.path.join(REF_GOLDEN_DIR, request.module.__name__ + ".json")
+        self.key = request.node.name
+        if self.path not in RefGolden._files:
+            RefGolden._files[self.path] = json.load(open(self.path)) if os.path.exists(self.path) else {}
+        self.table = RefGolden._files[self.path]
+        if RECORD:
+            assert have_ref(), "WM_RECORD_REF_GOLDEN=1 needs oracle/_ref (oracle/build_ref.sh)"
+            self.table[self.key] = []
+        assert self.key in self.table, f"no recorded reference results for {self.key} in {self.path}"
+        self.want, self.i = self.table[self.key], 0
+
+    def expect(self, ref_fn):
+        """The digest of the reference's answer to the next call."""
+        if RECORD:
+            self.want.append(digest(ref_fn()))
+            os.makedirs(REF_GOLDEN_DIR, exist_ok=True)
+            with open(self.path, "w") as f:
+                json.dump(self.table, f, indent=0, sort_keys=True)
+        assert self.i < len(self.want), f"{self.key}: more calls than the {len(self.want)} recorded"
+        self.i += 1
+        return self.want[self.i - 1]
+
+    def check(self, ref_fn, got, msg=""):
+        want = self.expect(ref_fn)
+        assert digest(got) == want, (f"{self.key}: call {self.i - 1} differs from the reference", msg)
+
+    def done(self):
+        assert self.i == len(self.want), f"{self.key}: {self.i} calls, {len(self.want)} recorded"
 
 
 def ref():

@@ -87,33 +87,80 @@ def test_gpu_map_batch_matches_golden(name, tmp_path):
     mp.close()
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
+def _flat_index(k, w, names, seq_len, seq_off, S, keys, pos_off, pos, bloom_bits, bloom):
+    """The arrays of an index view, keys in ascending order (what ref_idx_build_flat returns) and S without padding words:
+    equal indexes give equal digests."""
+    order = np.argsort(keys, kind="stable")
+    cnt = np.diff(pos_off.astype(np.int64))[order]
+    pos_sorted = np.concatenate([pos[int(pos_off[i]):int(pos_off[i + 1])] for i in order]) if len(order) else pos[:0]
+    s_words = (int(seq_len.astype(np.uint64).sum()) + 7) // 8
+    return (int(k), int(w), [bytes(n) for n in names], seq_len.astype(np.uint32), seq_off.astype(np.uint64), S[:s_words].astype(np.uint32),
+            keys[order].astype(np.uint64), cnt, pos_sorted.astype(np.uint64), int(bloom_bits), bloom[:int(bloom_bits) // 8].astype(np.uint8))
+
+
+def _blob_arrays(blob):
+    """The sections of wm_idx_blob_write's buffer (csrc/capi_map.cu): header, seq_len, seq_offset, names, S, keys, pos_off, pos, bloom."""
+    h = blob[:64].view(np.uint64)
+    n_seq, n_names, s_words, n_keys, n_pos, bloom_bits = (int(x) for x in h[2:8])
+    p = [64]
+
+    def take(nbytes, dtype):  # every section starts 8-byte aligned
+        a = blob[p[0]:p[0] + nbytes].view(dtype)
+        p[0] += (nbytes + 7) & ~7
+        return a
+    seq_len, seq_off = take(4 * n_seq, np.uint32), take(8 * n_seq, np.uint64)
+    names = take(n_names, np.uint8).tobytes().split(b"\0")[:n_seq]
+    S, keys = take(4 * s_words, np.uint32), take(8 * n_keys, np.uint64)
+    pos_off, pos = take(8 * (n_keys + 1), np.uint64), take(8 * n_pos, np.uint64)
+    return int(h[1] >> np.uint64(32)), int(h[1] & np.uint64(0xffffffff)), names, seq_len, seq_off, S, keys, pos_off, pos, bloom_bits, take(bloom_bits // 8, np.uint8)
+
+
 @pytest.mark.parametrize("name", ["ont_tandem", "asm20_small"])
-def test_idx_upload_from_the_reference_index(name, tmp_path):
+def test_idx_upload_from_the_reference_index(name, tmp_path, request):
     """The reference builds its own mm_idx_t (mm_idx_reader_read); the bucket walk of INTEGRATION.md section 3 flattens it;
-    wm_gpu_idx_upload takes the view; mapping through that context reproduces the golden PAF."""
-    from winnowmap_b200.mapper import make_options
+    wm_gpu_idx_upload takes the view; mapping through that context reproduces the golden PAF.  Where the reference is not
+    built the view is the library's own index (wm_idx_blob_write), which must equal the reference's flattened index: its
+    digest is recorded under tests/golden/ref/ (oracle_lib.RefGolden)."""
+    from winnowmap_b200.mapper import Mapper, make_options
+    g = ol.RefGolden(request)
     L = _lib()
-    R = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_harness.so"))
-    R.ref_idx_build_flat.restype = C.c_void_p
-    R.ref_idx_build_flat.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_int]
-    for f in ("keys", "pos_off", "pos", "S", "seq_len", "seq_off", "names", "bloom"):
-        getattr(R, "ref_idx_flat_" + f).restype = C.c_void_p
-        getattr(R, "ref_idx_flat_" + f).argtypes = [C.c_void_p]
-    R.ref_idx_flat_sizes.argtypes = [C.c_void_p, C.c_void_p]
-    R.ref_idx_flat_free.argtypes = [C.c_void_p]
     m = MANIFEST[name]
     ref, reads, wfile = make_golden.make_inputs(name, str(tmp_path))
     io, mo = make_options(m["params"]["preset"], True)
-    h = R.ref_idx_build_flat(ref.encode(), wfile.encode() if wfile else None, io.w, io.k, 3)
-    assert h
-    sz = np.zeros(7, np.uint64); R.ref_idx_flat_sizes(h, sz.ctypes.data)
-    v = IdxView(int(sz[5]), int(sz[6]), int(sz[0]), C.cast(R.ref_idx_flat_names(h), C.POINTER(C.c_char_p)), R.ref_idx_flat_seq_len(h),
-                R.ref_idx_flat_seq_off(h), R.ref_idx_flat_S(h), int(sz[1]), int(sz[2]), R.ref_idx_flat_keys(h), R.ref_idx_flat_pos_off(h),
-                R.ref_idx_flat_pos(h), int(sz[4]), R.ref_idx_flat_bloom(h))
+    if ol.RECORD:
+        R = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_harness.so"))
+        R.ref_idx_build_flat.restype = C.c_void_p
+        R.ref_idx_build_flat.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.c_int, C.c_int]
+        for f in ("keys", "pos_off", "pos", "S", "seq_len", "seq_off", "names", "bloom"):
+            getattr(R, "ref_idx_flat_" + f).restype = C.c_void_p
+            getattr(R, "ref_idx_flat_" + f).argtypes = [C.c_void_p]
+        R.ref_idx_flat_sizes.argtypes = [C.c_void_p, C.c_void_p]
+        R.ref_idx_flat_free.argtypes = [C.c_void_p]
+        h = R.ref_idx_build_flat(ref.encode(), wfile.encode() if wfile else None, io.w, io.k, 3)
+        assert h
+        sz = np.zeros(7, np.uint64); R.ref_idx_flat_sizes(h, sz.ctypes.data)
+
+        def arr(ptr, n, ct):
+            return np.ctypeslib.as_array(C.cast(ptr, C.POINTER(ct)), shape=(int(n),)).copy() if n else np.zeros(0, np.dtype(ct))
+        nm = C.cast(R.ref_idx_flat_names(h), C.POINTER(C.c_char_p))
+        flat = _flat_index(sz[5], sz[6], [nm[i] for i in range(int(sz[0]))], arr(R.ref_idx_flat_seq_len(h), sz[0], C.c_uint32),
+                           arr(R.ref_idx_flat_seq_off(h), sz[0], C.c_uint64), arr(R.ref_idx_flat_S(h), sz[1], C.c_uint32),
+                           arr(R.ref_idx_flat_keys(h), sz[2], C.c_uint64), arr(R.ref_idx_flat_pos_off(h), int(sz[2]) + 1, C.c_uint64),
+                           arr(R.ref_idx_flat_pos(h), sz[3], C.c_uint64), sz[4], arr(R.ref_idx_flat_bloom(h), int(sz[4]) // 8, C.c_uint8))
+        R.ref_idx_flat_free(h)
+    else:
+        mp = Mapper(ref, wfile, preset=m["params"]["preset"], cigar=True)
+        flat = _flat_index(*_blob_arrays(mp.index_blob()))
+        mp.close()
+    g.check(lambda: flat, flat)
+    g.done()
+    k, w, names, seq_len, seq_off, S, keys, cnt, pos, bloom_bits, bloom = flat
+    pos_off = np.concatenate([[0], np.cumsum(cnt)]).astype(np.uint64)
+    names_c = (C.c_char_p * len(names))(*names)
+    v = IdxView(k, w, len(names), C.cast(names_c, C.POINTER(C.c_char_p)), seq_len.ctypes.data, seq_off.ctypes.data, S.ctypes.data, len(S), len(keys), keys.ctypes.data,
+                pos_off.ctypes.data, pos.ctypes.data, bloom_bits, bloom.ctypes.data)
     ctx = L.wm_gpu_idx_upload(C.byref(v), 0)
-    assert ctx
-    R.ref_idx_flat_free(h)  # the library keeps its own copies
+    assert ctx  # the library keeps its own copies
     exp = gzip.open(os.path.join(ROOT, "tests", "golden", name + ".paf.gz")).read()
     out = str(tmp_path / "up.paf")
     _map_batch_paf(L, ctx, mo, _reads_in_print_order(reads), out)

@@ -140,18 +140,18 @@ def test_edge_case_reads_match_reference(key, sam, tmp_path):
 
 
 @pytest.mark.parametrize("preset,n50,err,n_reads", [("map-ont", 20000, 0.05, 2000), ("map-pb", 15000, 0.005, 1500)])
-def test_midsize_tandem_reference_matches_reference_binary(preset, n50, err, n_reads, tmp_path):
+def test_midsize_tandem_reference_matches_reference_binary(preset, n50, err, n_reads, tmp_path, request):
     """A 20 Mbp tandem-repeat-enriched reference (the 4-family rule of SURVEY.md 8d, -W list from the meryl rule) and a few
     thousand reads: multi-Mbase chunks on all orchestration lanes, giant chaining tasks, rl:i: > 0.  The expected output
-    comes from the reference binary itself (oracle/_ref/winnowmap, built from /root/reference by oracle/build_ref.sh and
-    shipped with the snapshot), run here on the same files."""
+    comes from the reference binary itself (oracle/_ref/winnowmap, built from the reference's sources by oracle/build_ref.sh)
+    run on the same files; its digest is recorded under tests/golden/ref/ (oracle_lib.RefGolden)."""
     import subprocess
     import numpy as np
     import gen_data
+    import oracle_lib as ol
     from winnowmap_b200.mapper import Mapper
+    g = ol.RefGolden(request)
     refbin = os.path.join(ROOT, "oracle", "_ref", "winnowmap")
-    if not os.path.exists(refbin):
-        pytest.skip("oracle/_ref/winnowmap not built")
     contigs = gen_data.make_ref(np.random.default_rng(1005), 20_000_000, 2, True)
     ref, reads, wf = str(tmp_path / "ref.fa"), str(tmp_path / "reads.fa"), str(tmp_path / "rep.txt")
     gen_data.write_fasta(ref, contigs)
@@ -159,17 +159,23 @@ def test_midsize_tandem_reference_matches_reference_binary(preset, n50, err, n_r
     assert n_w > 0
     recs = gen_data.make_reads(np.random.default_rng(2005), contigs, n_reads, n50, err, min_len=1000)
     gen_data.write_fasta(reads, recs)
-    exp_path = str(tmp_path / "ref.paf")
-    with open(exp_path, "wb") as f:
-        subprocess.run([refbin, "-t", str(os.cpu_count() or 4), "-c", "-x", preset, "-W", wf, ref, reads], stdout=f, stderr=subprocess.DEVNULL, check=True)
+
+    def reference_paf():
+        exp = subprocess.run([refbin, "-t", str(os.cpu_count() or 4), "-c", "-x", preset, "-W", wf, ref, reads], stdout=subprocess.PIPE,
+                             stderr=subprocess.DEVNULL, check=True).stdout
+        assert exp.count(b"\n") >= n_reads * 0.9
+        return exp
+    want = g.expect(reference_paf)
+    g.done()
     mp = Mapper(ref, wf, preset=preset, cigar=True)
     out = str(tmp_path / "out.paf")
     mp.map_file(reads, out)
     mp.close()
-    exp, got = open(exp_path, "rb").read(), open(out, "rb").read()
-    assert exp.count(b"\n") >= n_reads * 0.9
-    assert any(b"\trl:i:" in ln and not ln.rstrip().endswith(b"rl:i:0") for ln in exp.split(b"\n")[:4000]) or True
-    assert got == exp, _first_diff(exp, got)
+    got = open(out, "rb").read()
+    n_lines = got.count(b"\n")
+    assert n_lines >= n_reads * 0.9
+    assert any(b"\trl:i:" in ln and not ln.rstrip().endswith(b"rl:i:0") for ln in got.split(b"\n")[:4000]) or True
+    assert ol.digest(got) == want, f"output differs from the reference's ({n_lines} lines)"
 
 
 @pytest.mark.parametrize("key,sam,flags", [("paf_cs", 0, 0x40), ("paf_cs_long", 0, 0x40 | 0x800), ("sam_md", 1, 0x1000000),

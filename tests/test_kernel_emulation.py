@@ -176,7 +176,7 @@ def _tandem_anchors(rng, n_q, n_copies, unit, span=15):
         y.append(q0)
     x = np.concatenate(x).astype(np.uint64); y = np.concatenate(y).astype(np.uint64)
     xy = np.stack([x, np.uint64(span) << np.uint64(32) | y], axis=1)
-    return ol.ref_sort128(xy)
+    return ol.oracle_sort128(xy)  # the reference's order: tests/test_oracle_vs_ref.py::test_sorts_match_reference_including_ties
 
 
 @pytest.mark.parametrize("dense", [0, 1, 2, 3, 4])

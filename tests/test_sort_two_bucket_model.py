@@ -4,19 +4,15 @@ A radix pass of the reference (rs_sort, src/ksort.h:116-146) whose keys fall int
 a closed form: the misplaced elements of the lower bucket's region swap, in order, with the misplaced ones of the upper region, and the
 upper region shifts its own elements one slot to the right up to the last misplaced one.  Here the whole sort is restated in Python --
 serial cycle-leader walk for the other passes, the closed form for the two-bucket ones -- and compared with ref_radix_sort_128x
-(oracle/_ref, the reference's compiled code).  The CUDA implementation itself is checked on the GPU (tests/test_gpu_stages.py).
+(oracle/_ref, the reference's compiled code; its results on these seeded inputs are recorded under tests/golden/ref/).  The CUDA
+implementation itself is checked on the GPU (tests/test_gpu_stages.py).
 
 The second test checks the general form of the same observation (DESIGN.md section 8, not built as a kernel yet): the j-th element to
 arrive in a bucket ejects that bucket's j-th misplaced element, so the serial part of ANY pass is a token walk over the destination
 digits of the misplaced elements with one arrival counter per bucket; where each element lands follows from its arrival index."""
-import ctypes as C
-
 import numpy as np
-import pytest
 
 import oracle_lib as ol
-
-pytestmark = pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 
 
 def _walk(a, beg, end, s):
@@ -92,7 +88,8 @@ def _rs(a, beg, end, s, used):
                 _insertion(a, b[k], e[k])
 
 
-def test_two_bucket_closed_form_equals_the_reference_walk():
+def test_two_bucket_closed_form_equals_the_reference_walk(request):
+    g = ol.RefGolden(request)
     rng = np.random.default_rng(5)
     used = [0]
     for it in range(14):
@@ -103,15 +100,14 @@ def test_two_bucket_closed_form_equals_the_reference_walk():
         strand = (rng.random(n) < [0.0, 0.01, 0.5][it % 3]).astype(np.uint64)
         x = (strand << np.uint64(63)) | (np.uint64(it % 2) << np.uint64(32)) | pos
         a = np.ascontiguousarray(np.stack([x, np.arange(n, dtype=np.uint64)], axis=1))
-        ref = a.copy()
-        ol.ref().ref_radix_sort_128x(ref.ctypes.data_as(C.POINTER(C.c_uint64)), n)
         got = a.copy()
         if n <= 64:
             _insertion(got, 0, n)
         else:
             _rs(got, 0, n, 56, used)
-        assert np.array_equal(got, ref), (it, n)
+        g.check(lambda: ol.ref_sort128(a), got, (it, n))
     assert used[0] >= 10
+    g.done()
 
 
 def _token_pass(a, beg, end, s, steps):
@@ -161,7 +157,8 @@ def _rs_token(a, beg, end, s, steps):
                 _insertion(a, b[k], e[k])
 
 
-def test_token_walk_formulation_equals_the_reference_sort():
+def test_token_walk_formulation_equals_the_reference_sort(request):
+    g = ol.RefGolden(request)
     rng = np.random.default_rng(11)
     for it in range(10):
         n = int(rng.choice([100, 400, 1500, 4000]))
@@ -171,9 +168,8 @@ def test_token_walk_formulation_equals_the_reference_sort():
         strand = (rng.random(n) < [0.0, 0.02, 0.5][it % 3]).astype(np.uint64)
         x = (strand << np.uint64(63)) | (np.uint64(rng.integers(0, 3)) << np.uint64(32)) | pos
         a = np.ascontiguousarray(np.stack([x, np.arange(n, dtype=np.uint64)], axis=1))
-        ref = a.copy()
-        ol.ref().ref_radix_sort_128x(ref.ctypes.data_as(C.POINTER(C.c_uint64)), n)
         got, steps = a.copy(), [0]
         _rs_token(got, 0, n, 56, steps)
-        assert np.array_equal(got, ref), (it, n)
+        g.check(lambda: ol.ref_sort128(a), got, (it, n))
         assert steps[0] <= 2 * n  # serial steps of the whole sort: about 1.3 per element, against 2-3 walker steps per element today
+    g.done()

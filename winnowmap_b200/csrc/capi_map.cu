@@ -635,6 +635,20 @@ extern "C" int wm_bench_write(wm_gpu_ctx_s *c, const wm_mapopt_t *opt, int n_fir
 	return n;
 }
 
+// bench: the records of the last resident pass themselves, for reads [first, first + n) (output comparison of two builds)
+extern "C" int64_t wm_bench_records(const wm_gpu_ctx_s *c, int first, int n, int32_t *n_reg, int32_t *rep_len, wm_reg1_t *regs, int64_t cap)
+{
+	int64_t k = 0;
+	for (int i = first; i < first + n; ++i) {
+		const bool have = i >= 0 && i < (int)c->res_regs.size();
+		n_reg[i - first] = have ? (int32_t)c->res_regs[i].size() : 0;
+		rep_len[i - first] = have ? c->res_rl[i] : 0;
+		if (have)
+			for (const wm_reg1_t &r : c->res_regs[i]) { if (k < cap) regs[k] = r; ++k; }
+	}
+	return k;
+}
+
 // The records wm_gpu_map_batch returned, formatted in input order with the writer wm_map_file uses (mm_write_paf3 / mm_write_sam3)
 extern "C" int wm_format_batch(const wm_gpu_ctx_s *c, const wm_mapopt_t *opt, int n_seq, const char *const *names, const char *const *seqs, const int32_t *lens,
                                const int32_t *n_reg, wm_reg1_t *const *reg, const int32_t *rep_len, const char *out_fn)
