@@ -95,6 +95,8 @@ int wm_sketch_batch(const wm_bloom_t *bloom, int n, const char *seq, const int64
 /* radix_sort_128x (src/misc.c:156; src/ksort.h:116-151) on n_arr independent arrays:
  * array i is a[off[i] .. off[i+1]); sorted in place with the reference's tie order. */
 int wm_radix_sort_128x_batch(int n_arr, wm128_t *a, const int64_t *off);
+/* The same, also returning in *ms the device time of the sort alone (CUDA events; the copies are left out). */
+int wm_radix_sort_128x_batch_timed(int n_arr, wm128_t *a, const int64_t *off, float *ms);
 
 /* Batched mm_chain_dp (src/chain.c:22; prototype src/mmpriv.h:67) for n_segs = 1,
  * is_cdna = 0.  Anchors of task i: a[off[i] .. off[i+1]) (sorted as by collect_seed_hits).

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Tuning aid (GPU box): the tie-exact anchor sort on arrays shaped like the anchors of a read inside a tandem array
-(concatenated ascending runs, many equal keys).  Run under ncu to see the kernel times:
+(concatenated ascending runs, many equal keys).  Prints the wall time of one call and the device time of the sort alone (CUDA
+events, copies left out).  Run under ncu to see the kernel times:
    ncu --metrics gpu__time_duration.sum --csv --log-file x.csv python tools/bench_sort.py --n 30000 --arrays 200"""
 import argparse
 import os
@@ -35,6 +36,7 @@ def main():
     ap.add_argument("--arrays", type=int, default=200)
     ap.add_argument("--check", action="store_true")
     ap.add_argument("--strand-frac", type=float, default=0.0)
+    ap.add_argument("--repeat", type=int, default=5, help="device-timed runs of the whole batch")
     a = ap.parse_args()
     from winnowmap_b200 import kernels
     rng = np.random.default_rng(5)
@@ -44,6 +46,9 @@ def main():
     out = kernels.radix_sort_128x_batch(arrays)
     dt = time.time() - t0
     print(f"{a.arrays} arrays x {len(arrays[0])} anchors: {dt * 1e3:.1f} ms wall (incl. copies)")
+    dev = [kernels.radix_sort_128x_batch(arrays, timed=True)[1] for _ in range(a.repeat)]
+    print(f"{a.arrays} arrays x {len(arrays[0])} anchors: device ms of the sort (copies left out) median {np.median(dev):.2f} "
+          f"min {min(dev):.2f} max {max(dev):.2f} over {a.repeat} runs")
     if a.check:
         sys.path.insert(0, os.path.join(ROOT, "tests"))
         import oracle_lib as ol

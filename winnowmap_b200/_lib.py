@@ -48,6 +48,7 @@ def lib():
         L.wm_sketch_batch.argtypes = [C.c_void_p, C.c_int, C.c_char_p, i64p, u32p, C.c_int, C.c_int,
                                       C.POINTER(C.c_void_p), C.POINTER(C.c_void_p)]
         L.wm_radix_sort_128x_batch.argtypes = [C.c_int, u64p, i64p]
+        L.wm_radix_sort_128x_batch_timed.argtypes = [C.c_int, u64p, i64p, C.POINTER(C.c_float)]
         L.wm_chain_dp_batch.argtypes = [C.c_int, u64p, i64p] + [C.c_int] * 8 + [C.c_float, i32p, u64p, u64p, i64p]
         _lib = L
     return _lib

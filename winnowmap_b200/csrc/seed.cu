@@ -184,6 +184,9 @@ struct wm_gs_sm {
 	int b[256];                    // write pointers (walker)
 	int filled[256];               // originals loaded so far, per bucket (feeders)
 	int hist[256];
+	int moff[257];                 // token pass: offsets of every bucket's misplaced slots in the list
+	int A[256];                    // token pass: arrivals in every bucket before its own turn
+	int wtot[4];                   // per-warp totals of wm_gs_block_excl
 	int n_big, n_small, next_small, walk_done;
 	wm_rs_warp_ws W[4];
 	wm_rs_range swl[4][40];        // per-warp work list of phase 2 (disjoint sub-ranges of > 64 elements of a <= 2048-element range)
@@ -274,17 +277,196 @@ __device__ void wm_gs_two_bucket_pass(wm128_dev *a, wm128_dev *tmp, int32_t *idx
 	__syncthreads();
 }
 
+// ---- a pass with three or more non-empty buckets: a token walk over destination digits ----
+// The j-th element to arrive in a bucket ejects that bucket's j-th misplaced element (a slot of its region holding another bucket's
+// element).  So the serial part of the walk needs only the destination digits D of the misplaced elements, listed in slot order
+// (hence grouped by the bucket that owns the slot: bucket k's at list indices [moff[k], moff[k+1])), and one arrival pointer per
+// bucket.  Bucket k's turn opens a cycle at each of its list entries not yet ejected; the element in hand arrives at index
+// p = ptr[t]++ of its bucket t's list and the element listed there is next in hand, until one whose digit is k closes the cycle.
+// No 16-byte element moves during the walk: land[] records, per list index, an arrival index p or ~opener, and the elements are
+// then placed by all threads with index arithmetic:
+//   - an arrival at index p of bucket t lands at the start of run p - moff[t] of t (B[t], or one past the previous misplaced slot);
+//   - the element closing a cycle lands in the slot where the cycle was opened;
+//   - an element already in its region moves one slot to the right if its run r has r < A[t] (the arrivals in t before t's turn
+//     emptied those runs' misplaced slots), and stays otherwise.
+// tests/test_sort_token_walk.py restates this in the same flat form and checks it against the serial walk.
+// Scratch: the list's slots M in tmp (as int32), land[] in idx.  D is staged in shared memory (the FIFO / stage union) when the list
+// fits there; otherwise it stays in idx as int32 (land[] overwrites it after use) and the three feeder warps stream it to the walker
+// through per-bucket byte FIFOs -- the walker consumes every bucket's list in order, as it consumes the element FIFOs.
+__device__ __forceinline__ int wm_gs_owner(const int *E, int i)
+{ // smallest k with E[k] > i (E non-decreasing, E[255] > i): the bucket whose region holds slot i
+	int k = 0;
+	#pragma unroll
+	for (int w = 128; w > 0; w >>= 1) if (E[k + w - 1] <= i) k += w;
+	return k;
+}
+
+__device__ __forceinline__ int wm_gs_byte_read(const unsigned char *p)
+{ // (volatile: stays ahead of the store of the arrival pointer that frees the FIFO entry)
+	uint32_t r;
+	asm volatile("ld.shared.u8 %0, [%1];" : "=r"(r) : "r"((uint32_t)__cvta_generic_to_shared(p)));
+	return (int)r;
+}
+
+template <bool WM_GS_DBG, typename sm_t>
+__device__ void wm_gs_token_pass(sm_t *S, wm128_dev *a, wm128_dev *tmp, int32_t *idx, int beg, int end, int s, int tid,
+                                 unsigned long long &n_steps, unsigned long long &n_wait, bool &byte_fifo)
+{
+	constexpr int DCAP = (int)sizeof(S->u); // digits that fit in shared memory
+	constexpr int FB = DCAP / 256;          // byte FIFO depth per bucket
+	int *M = (int*)(tmp + beg);
+	int32_t *land = idx + beg;
+	unsigned char *Ds = (unsigned char*)&S->u;
+	const int lane = tid & 31, wid = tid >> 5;
+	// 1. the list: slots, digits, and its length per bucket
+	for (int k = tid; k < 256; k += WM_GS_THREADS) S->hist[k] = 0;
+	__syncthreads();
+	int carry = 0, tot;
+	for (int base = beg; base < end; base += WM_GS_THREADS) {
+		const int i = base + tid;
+		int own = 0, d = 0;
+		if (i < end) { own = wm_gs_owner(S->E, i); d = (int)(a[i].x >> s & 255); }
+		const bool flag = i < end && d != own;
+		const int g = carry + wm_gs_block_excl(flag, S->wtot, tid, &tot);
+		const unsigned peers = __match_any_sync(0xffffffffu, flag ? own : 256 + lane);
+		if (flag) {
+			M[g] = i, land[g] = d;
+			if (g < DCAP) Ds[g] = (unsigned char)d;
+			if (lane == __ffs(peers) - 1) atomicAdd(&S->hist[own], __popc(peers));
+		}
+		carry += tot;
+	}
+	const int m = carry;
+	const bool staged = m <= DCAP;
+	byte_fifo = !staged;
+	__syncthreads();
+	if (wid == 0) { // list offsets; the arrival pointers b[] and the feeders' marks filled[] start there
+		int cnt[8], sum = 0;
+		#pragma unroll
+		for (int k = 0; k < 8; ++k) { cnt[k] = S->hist[lane * 8 + k]; sum += cnt[k]; }
+		int incl = sum;
+		#pragma unroll
+		for (int o = 1; o < 32; o <<= 1) { int t2 = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t2; }
+		int acc = incl - sum;
+		#pragma unroll
+		for (int k = 0; k < 8; ++k) { S->moff[lane * 8 + k] = acc; S->b[lane * 8 + k] = acc; S->filled[lane * 8 + k] = acc; acc += cnt[k]; }
+		if (lane == 31) S->moff[256] = acc;
+		if (lane == 0) S->walk_done = 0;
+	}
+	__syncthreads();
+	// 2. the walk
+	if (tid == 0) {
+		int *ptr = S->b; const int *moff = S->moff;
+		if (staged) {
+			for (int k = 0; k < 256; ++k) {
+				int f = ptr[k]; // (no arrivals in k during its own turn: ptr[k] stays)
+				const int fe = moff[k + 1];
+				S->A[k] = f - moff[k];
+				for (; f < fe; ++f) {
+					int cur = f, t = Ds[f];
+					for (;;) {
+						const int p = ptr[t];
+						ptr[t] = p + 1;
+						land[cur] = p;
+						const int t2 = Ds[p];
+						if (WM_GS_DBG) ++n_steps;
+						if (t2 == k) { land[p] = ~f; break; }
+						cur = p, t = t2;
+					}
+				}
+			}
+		} else {
+			volatile int *filled = S->filled;
+			for (int k = 0; k < 256; ++k) {
+				int f = ptr[k];
+				const int fe = moff[k + 1];
+				S->A[k] = f - moff[k];
+				while (f < fe) {
+					const int opener = f;
+					while (filled[k] <= f) { if (WM_GS_DBG) ++n_wait; }
+					int t = wm_gs_byte_read(&Ds[k * FB + (f & (FB - 1))]);
+					*(volatile int*)&ptr[k] = ++f;
+					int cur = opener;
+					for (;;) {
+						const int p = ptr[t];
+						while (filled[t] <= p) { if (WM_GS_DBG) ++n_wait; }
+						const int t2 = wm_gs_byte_read(&Ds[t * FB + (p & (FB - 1))]);
+						*(volatile int*)&ptr[t] = p + 1;
+						land[cur] = p;
+						if (WM_GS_DBG) ++n_steps;
+						if (t2 == k) { land[p] = ~opener; break; }
+						cur = p, t = t2;
+					}
+				}
+			}
+		}
+		__threadfence_block();
+		*(volatile int*)&S->walk_done = 1;
+	} else if (!staged && wid > 0) { // feeders: 96 threads, buckets tid - 32, + 96, + 192
+		volatile int *bv = S->b; volatile int *done = &S->walk_done;
+		for (;;) {
+			bool any = false, fed = false;
+			for (int k = tid - 32; k < 256; k += WM_GS_THREADS - 32) {
+				const int fl = S->filled[k], ek = S->moff[k + 1];
+				if (fl >= ek) continue;
+				any = true;
+				const int want = ek - fl < 16 ? ek - fl : 16;
+				if (FB - (fl - bv[k]) >= want) {
+					int r[16];
+					#pragma unroll
+					for (int q = 0; q < 16; ++q) if (q < want) r[q] = land[fl + q];
+					#pragma unroll
+					for (int q = 0; q < 16; ++q) if (q < want) Ds[k * FB + ((fl + q) & (FB - 1))] = (unsigned char)r[q];
+					__threadfence_block();
+					*(volatile int*)&S->filled[k] = fl + want;
+					fed = true;
+				}
+			}
+			if (!any || *done) break;
+			if (!fed) __nanosleep(256);
+		}
+	}
+	__syncthreads();
+	// 3. where every listed element lands (M is read here for the last time)
+	for (int f = tid; f < m; f += WM_GS_THREADS) {
+		const int L = land[f];
+		int dst;
+		if (L < 0) dst = M[~L];
+		else { const int t = wm_gs_owner(S->moff + 1, L); dst = L == S->moff[t] ? S->B[t] : M[L - 1] + 1; }
+		land[f] = dst;
+	}
+	__syncthreads();
+	// 4. placement into tmp, and back
+	carry = 0;
+	for (int base = beg; base < end; base += WM_GS_THREADS) {
+		const int i = base + tid;
+		wm128_dev e; e.x = e.y = 0;
+		int own = 0;
+		if (i < end) { e = a[i]; own = wm_gs_owner(S->E, i); }
+		const bool flag = i < end && (int)(e.x >> s & 255) != own;
+		const int g = carry + wm_gs_block_excl(flag, S->wtot, tid, &tot);
+		if (i < end) tmp[flag ? land[g] : (g - S->moff[own] < S->A[own] ? i + 1 : i)] = e;
+		carry += tot;
+	}
+	__syncthreads();
+	for (int t = beg + tid; t < end; t += WM_GS_THREADS) a[t] = tmp[t];
+	__syncthreads();
+}
+
 template <int WM_GS_F, int WM_GS_STAGE, bool WM_GS_DBG>
 __global__ void __launch_bounds__(WM_GS_THREADS)
 wm_anchor_sort_giant_kernel(wm128_dev *__restrict__ a_all, const int64_t *__restrict__ off, const int32_t *__restrict__ ids, int n_arr,
-                            wm_rs_range *__restrict__ wl_all, unsigned long long *dbg, wm128_dev *__restrict__ tmp_all, int32_t *__restrict__ idx_all, int two_min)
+                            wm_rs_range *__restrict__ wl_all, unsigned long long *dbg, wm128_dev *__restrict__ tmp_all, int32_t *__restrict__ idx_all,
+                            const int64_t *__restrict__ scr_off, int two_min, int token_min)
 {
-	// tmp_all / idx_all: scratch of the closed-form pass (wm_gs_two_bucket_pass), indexed like a_all; two_min: ranges of at least this many
-	// elements take it when their pass has two non-empty buckets (0: never)
-	// dbg (tuning aid, WM_SORT_DEBUG=1): clocks spent by thread 0 in [0] histograms, [1] the walk, [2] sub-bucket dispatch + tiny sorts,
-	// [3] phase 2, [4] walker steps, [5] walker waits (polls of an empty FIFO)
+	// tmp_all / idx_all: scratch of the closed-form and token passes (one element + one int32 per anchor); array ai's slice starts at
+	// scr_off[ai] and is indexed like the array.  two_min / token_min: ranges of at least this many elements take the closed form when
+	// their pass has two non-empty buckets / the token walk when it has more (0: never)
+	// dbg (tuning aid, WM_SORT_DEBUG=1): clocks spent by thread 0 in [0] histograms, [1] the walk (any pass kind), [2] sub-bucket
+	// dispatch + tiny sorts, [3] phase 2, [4] walker steps, [5] walker waits (polls of an empty FIFO), [6] elements in closed-form
+	// passes, [7] token-walk steps, [8] elements in token passes, [9] token passes fed through byte FIFOs
 	long long t_dbg = dbg ? clock64() : 0;
-	unsigned long long n_steps_dbg = 0, n_wait_dbg = 0;
+	unsigned long long n_steps_dbg = 0, n_wait_dbg = 0, n_tok_dbg = 0;
 #define WM_GS_LAP(i) do { if (dbg && tid == 0) { const long long t2 = clock64(); atomicAdd(dbg + (i), (unsigned long long)(t2 - t_dbg)); t_dbg = t2; } } while (0)
 	extern __shared__ __align__(16) unsigned char wm_gs_smem[];
 	typedef wm_gs_sm<WM_GS_F, WM_GS_STAGE> sm_t;
@@ -297,6 +479,8 @@ wm_anchor_sort_giant_kernel(wm128_dev *__restrict__ a_all, const int64_t *__rest
 		const int64_t base = off[task];
 		const int n = (int)(off[task + 1] - base);
 		wm128_dev *a = a_all + base;
+		wm128_dev *tmp = scr_off ? tmp_all + scr_off[ai] : 0;
+		int32_t *idx = scr_off ? idx_all + scr_off[ai] : 0;
 		asm volatile("" : "+l"(a)); // keep the pointer in registers: the walker's loop was re-deriving it from the parameter bank (an LDC per step)
 		// work lists in global memory (the array's slice of wl_all: n / 64 + 1 entries): big ranges grow from the front,
 		// small ones from the back
@@ -344,8 +528,12 @@ wm_anchor_sort_giant_kernel(wm128_dev *__restrict__ a_all, const int64_t *__rest
 			}
 			__syncthreads();
 			if (n_nz == 2 && two_min > 0 && end - beg >= two_min) { // two buckets: the pass in closed form, by all threads
-				wm_gs_two_bucket_pass(a, tmp_all + base, idx_all + base, beg, S->E[lo_digit], end, s, lo_digit, S->hist, tid);
+				wm_gs_two_bucket_pass(a, tmp, idx, beg, S->E[lo_digit], end, s, lo_digit, S->hist, tid);
 				if (WM_GS_DBG && tid == 0) atomicAdd(dbg + 6, (unsigned long long)(end - beg));
+			} else if (n_nz > 2 && token_min > 0 && end - beg >= token_min) { // the token walk, placement by all threads
+				bool byte_fifo;
+				wm_gs_token_pass<WM_GS_DBG>(S, a, tmp, idx, beg, end, s, tid, n_tok_dbg, n_wait_dbg, byte_fifo);
+				if (WM_GS_DBG && tid == 0) { atomicAdd(dbg + 8, (unsigned long long)(end - beg)); if (byte_fifo) atomicAdd(dbg + 9, 1ULL); }
 			} else
 			if (tid == 0) { // the walker (ksort.h:126-138); b[] are its pointers, filled[] the feeders'
 				volatile int *filled = S->filled; int *b = S->b; const int *E = S->E;
@@ -445,7 +633,7 @@ wm_anchor_sort_giant_kernel(wm128_dev *__restrict__ a_all, const int64_t *__rest
 		__syncthreads();
 		WM_GS_LAP(3);
 	}
-	if (dbg && tid == 0) { atomicAdd(dbg + 4, n_steps_dbg); atomicAdd(dbg + 5, n_wait_dbg); }
+	if (dbg && tid == 0) { atomicAdd(dbg + 4, n_steps_dbg); atomicAdd(dbg + 5, n_wait_dbg); atomicAdd(dbg + 7, n_tok_dbg); }
 #undef WM_GS_LAP
 }
 
@@ -484,17 +672,30 @@ void wm_anchor_sort_run(wm_seed_ws *ws, wm128_dev *d_a, const int64_t *d_off, co
 		while (n_l < big.size() && h_off[big[n_l] + 1] - h_off[big[n_l]] > cap_m) ++n_l;
 		while (n_l + n_m < big.size() && h_off[big[n_l + n_m] + 1] - h_off[big[n_l + n_m]] > cap_s) ++n_m;
 		const size_t n_s = big.size() - n_l - n_m;
-		int32_t *d_big = (int32_t*)ws->big_ids.need(sizeof(int32_t) * big.size());
-		wm_rs_range *d_wl = (wm_rs_range*)ws->rs_stacks.need(sizeof(wm_rs_range) * (size_t)((h_off[n_arr] >> 6) + n_arr + 2));
-		WM_CUDA_CHECK(wm_memcpy_async(d_big, big.data(), sizeof(int32_t) * big.size(), cudaMemcpyHostToDevice, st));
-		// scratch of the closed-form two-bucket passes of the walker kernels (one element + one int32 per anchor)
+		// scratch of the closed-form and token passes of the walker kernels: one element + one int32 per anchor of the arrays they sort,
+		// array big[q] (q < n_l + n_m) at scratch offset scr[q]
 		static int two_min = -1; // WM_SORT_TWO_MIN: ranges of at least this many anchors take the closed form (0: always walk)
 		if (two_min < 0) { const char *e = getenv("WM_SORT_TWO_MIN"); two_min = e ? atoi(e) : 512; }
+		static int token_min = -1; // WM_SORT_TOKEN_MIN: ranges of at least this many anchors take the token walk (0: always the element walker)
+		if (token_min < 0) { const char *e = getenv("WM_SORT_TOKEN_MIN"); token_min = e ? atoi(e) : 512; }
+		const size_t n_w = n_l + n_m;
+		std::vector<int64_t> scr(n_w + 1, 0);
+		for (size_t q = 0; q < n_w; ++q) scr[q + 1] = scr[q] + (h_off[big[q] + 1] - h_off[big[q]]);
+		const bool use_scr = (two_min > 0 || token_min > 0) && n_w > 0;
+		// device copies: scratch offsets (int64, first for alignment), then the array ids
+		int64_t *d_scr = (int64_t*)ws->big_ids.need(sizeof(int64_t) * (n_w + 1) + sizeof(int32_t) * big.size());
+		int32_t *d_big = (int32_t*)(d_scr + n_w + 1);
+		wm_rs_range *d_wl = (wm_rs_range*)ws->rs_stacks.need(sizeof(wm_rs_range) * (size_t)((h_off[n_arr] >> 6) + n_arr + 2));
+		WM_CUDA_CHECK(wm_memcpy_async(d_big, big.data(), sizeof(int32_t) * big.size(), cudaMemcpyHostToDevice, st));
 		wm128_dev *d_tmp = 0; int32_t *d_idx = 0;
-		if (two_min > 0 && (n_l || n_m)) {
-			d_tmp = (wm128_dev*)ws->sort_tmp.need(sizeof(wm128_dev) * (size_t)(h_off[n_arr] + 1));
-			d_idx = (int32_t*)ws->sort_idx.need(sizeof(int32_t) * (size_t)(h_off[n_arr] + 1));
+		if (use_scr) {
+			WM_CUDA_CHECK(wm_memcpy_async(d_scr, scr.data(), sizeof(int64_t) * (n_w + 1), cudaMemcpyHostToDevice, st));
+			d_tmp = (wm128_dev*)ws->sort_tmp.need(sizeof(wm128_dev) * (size_t)(scr[n_w] + 1));
+			d_idx = (int32_t*)ws->sort_idx.need(sizeof(int32_t) * (size_t)(scr[n_w] + 1));
 		}
+		const int64_t *d_scr_l = use_scr ? d_scr : 0, *d_scr_m = use_scr ? d_scr + n_l : 0;
+		const char *dbg_fmt = "[sort-debug] arrays=%d clocks: hist %llu walk %llu dispatch %llu phase2 %llu | walker steps %llu wait polls %llu | "
+		                      "elements in closed-form passes %llu | token-walk steps %llu elements in token passes %llu byte-FIFO passes %llu\n";
 		if (n_l) {
 			wm_count_launch();
 			if (giant) {
@@ -506,17 +707,17 @@ void wm_anchor_sort_run(wm_seed_ws *ws, wm128_dev *d_a, const int64_t *d_off, co
 					attr_set = true;
 				}
 				unsigned long long *dbg = 0;
-				if (getenv("WM_SORT_DEBUG")) { WM_CUDA_CHECK(cudaMalloc((void**)&dbg, 64)); WM_CUDA_CHECK(cudaMemset(dbg, 0, 64)); }
+				if (getenv("WM_SORT_DEBUG")) { WM_CUDA_CHECK(cudaMalloc((void**)&dbg, 128)); WM_CUDA_CHECK(cudaMemset(dbg, 0, 128)); }
 				static int giant_ctas = -1; // WM_SORT_GIANT_CTAS
 				if (giant_ctas < 0) { const char *e = getenv("WM_SORT_GIANT_CTAS"); giant_ctas = e && atoi(e) > 0 ? atoi(e) : 148; }
 				const unsigned g_l = (unsigned)(n_l < (size_t)giant_ctas ? n_l : (size_t)giant_ctas);
-				if (dbg) wm_anchor_sort_giant_kernel<16, 2048, true><<<g_l, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big, (int)n_l, d_wl, dbg, d_tmp, d_idx, two_min);
-				else wm_anchor_sort_giant_kernel<16, 2048, false><<<g_l, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big, (int)n_l, d_wl, 0, d_tmp, d_idx, two_min);
+				if (dbg) wm_anchor_sort_giant_kernel<16, 2048, true><<<g_l, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big, (int)n_l, d_wl, dbg, d_tmp, d_idx, d_scr_l, two_min, token_min);
+				else wm_anchor_sort_giant_kernel<16, 2048, false><<<g_l, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big, (int)n_l, d_wl, 0, d_tmp, d_idx, d_scr_l, two_min, token_min);
 				if (dbg) {
-					unsigned long long h[8];
+					unsigned long long h[16];
 					WM_CUDA_CHECK(cudaStreamSynchronize(st));
-					WM_CUDA_CHECK(cudaMemcpy(h, dbg, 64, cudaMemcpyDeviceToHost));
-					fprintf(stderr, "[sort-debug] arrays=%d clocks: hist %llu walk %llu dispatch %llu phase2 %llu | walker steps %llu wait polls %llu | elements in closed-form passes %llu\n", (int)n_l, h[0], h[1], h[2], h[3], h[4], h[5], h[6]);
+					WM_CUDA_CHECK(cudaMemcpy(h, dbg, 128, cudaMemcpyDeviceToHost));
+					fprintf(stderr, dbg_fmt, (int)n_l, h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], h[8], h[9]);
 					cudaFree(dbg);
 				}
 			} else wm_anchor_sort_big_kernel<<<(unsigned)n_l, 32, 0, st>>>(d_a, d_off, d_big, (int)n_l, d_wl, 0);
@@ -532,18 +733,18 @@ void wm_anchor_sort_run(wm_seed_ws *ws, wm128_dev *d_a, const int64_t *d_off, co
 					attr_set = true;
 				}
 				unsigned long long *dbg = 0;
-				if (getenv("WM_SORT_DEBUG")) { WM_CUDA_CHECK(cudaMalloc((void**)&dbg, 64)); WM_CUDA_CHECK(cudaMemset(dbg, 0, 64)); }
+				if (getenv("WM_SORT_DEBUG")) { WM_CUDA_CHECK(cudaMalloc((void**)&dbg, 128)); WM_CUDA_CHECK(cudaMemset(dbg, 0, 128)); }
 				static int med_ctas = -1; // WM_SORT_MEDIUM_CTAS: resident CTAs of the medium class (47 KB of shared memory each)
 				if (med_ctas < 0) { const char *e = getenv("WM_SORT_MEDIUM_CTAS"); med_ctas = e && atoi(e) > 0 ? atoi(e) : 592; }
 				const unsigned g_m = (unsigned)(n_m < (size_t)med_ctas ? n_m : (size_t)med_ctas);
 				if (dbg) {
-					wm_anchor_sort_giant_kernel<8, 512, true><<<g_m, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big + n_l, (int)n_m, d_wl, dbg, d_tmp, d_idx, two_min);
-					unsigned long long h[8];
+					wm_anchor_sort_giant_kernel<8, 512, true><<<g_m, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big + n_l, (int)n_m, d_wl, dbg, d_tmp, d_idx, d_scr_m, two_min, token_min);
+					unsigned long long h[16];
 					WM_CUDA_CHECK(cudaStreamSynchronize(st));
-					WM_CUDA_CHECK(cudaMemcpy(h, dbg, 64, cudaMemcpyDeviceToHost));
-					fprintf(stderr, "[sort-debug] arrays=%d clocks: hist %llu walk %llu dispatch %llu phase2 %llu | walker steps %llu wait polls %llu | elements in closed-form passes %llu\n", (int)n_m, h[0], h[1], h[2], h[3], h[4], h[5], h[6]);
+					WM_CUDA_CHECK(cudaMemcpy(h, dbg, 128, cudaMemcpyDeviceToHost));
+					fprintf(stderr, dbg_fmt, (int)n_m, h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], h[8], h[9]);
 					cudaFree(dbg);
-				} else wm_anchor_sort_giant_kernel<8, 512, false><<<g_m, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big + n_l, (int)n_m, d_wl, 0, d_tmp, d_idx, two_min);
+				} else wm_anchor_sort_giant_kernel<8, 512, false><<<g_m, WM_GS_THREADS, sizeof(sm_t), st>>>(d_a, d_off, d_big + n_l, (int)n_m, d_wl, 0, d_tmp, d_idx, d_scr_m, two_min, token_min);
 			} else wm_anchor_sort_big_kernel<<<(unsigned)n_m, 32, cap_m * sizeof(wm128_dev), st>>>(d_a, d_off, d_big + n_l, (int)n_m, d_wl, cap_m);
 		}
 		if (n_s) { wm_count_launch(); wm_anchor_sort_big_kernel<<<(unsigned)n_s, 32, cap_s * sizeof(wm128_dev), st>>>(d_a, d_off, d_big + n_l + n_m, (int)n_s, d_wl, cap_s); }
@@ -610,8 +811,8 @@ void wm_idx_dev_build_ht(wm_idx_dev *ix, cudaStream_t st)
 	ix->ht_key = hk, ix->ht_val = hv, ix->ht_mask = cap - 1;
 }
 
-// ---- C ABI: standalone tie-exact sort (for the parity tests) ----
-extern "C" int wm_radix_sort_128x_batch(int n_arr, wm128_dev *a, const int64_t *off)
+// ---- C ABI: standalone tie-exact sort (for the parity tests and tools/bench_sort.py) ----
+extern "C" int wm_radix_sort_128x_batch_timed(int n_arr, wm128_dev *a, const int64_t *off, float *ms)
 {
 	int ndev = 0;
 	if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
@@ -625,10 +826,19 @@ extern "C" int wm_radix_sort_128x_batch(int n_arr, wm128_dev *a, const int64_t *
 	WM_CUDA_CHECK(cudaMemcpy(d_a, a, sizeof(wm128_dev) * n, cudaMemcpyHostToDevice));
 	WM_CUDA_CHECK(cudaMemcpy(d_off, off, sizeof(int64_t) * (n_arr + 1), cudaMemcpyHostToDevice));
 	wm_seed_ws ws;
+	cudaEvent_t ev[2];
+	if (ms) { WM_CUDA_CHECK(cudaEventCreate(&ev[0])); WM_CUDA_CHECK(cudaEventCreate(&ev[1])); WM_CUDA_CHECK(cudaEventRecord(ev[0], 0)); }
 	wm_anchor_sort_run(&ws, d_a, d_off, off, n_arr, 0);
+	if (ms) WM_CUDA_CHECK(cudaEventRecord(ev[1], 0));
 	WM_CUDA_CHECK(cudaDeviceSynchronize());
+	if (ms) { WM_CUDA_CHECK(cudaEventElapsedTime(ms, ev[0], ev[1])); cudaEventDestroy(ev[0]); cudaEventDestroy(ev[1]); }
 	WM_CUDA_CHECK(cudaMemcpy(a, d_a, sizeof(wm128_dev) * n, cudaMemcpyDeviceToHost));
 	ws.release();
 	cudaFree(d_a); cudaFree(d_off);
 	return 0;
+}
+
+extern "C" int wm_radix_sort_128x_batch(int n_arr, wm128_dev *a, const int64_t *off)
+{
+	return wm_radix_sort_128x_batch_timed(n_arr, a, off, 0);
 }

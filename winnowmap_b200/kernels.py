@@ -142,15 +142,21 @@ def sketch_batch(bloom, seqs, w, k, rids=None):
     return [xy[o[i]: o[i + 1]].copy() for i in range(n)]
 
 
-def radix_sort_128x_batch(arrays):
-    """radix_sort_128x (reference src/misc.c:156) on each (n,2) uint64 array, tie order included."""
+def radix_sort_128x_batch(arrays, timed=False):
+    """radix_sort_128x (reference src/misc.c:156) on each (n,2) uint64 array, tie order included.
+    timed=True: returns (sorted arrays, device milliseconds of the sort alone, copies left out)."""
     n = len(arrays)
     off = np.zeros(n + 1, dtype=np.int64)
     if n:
         off[1:] = np.cumsum([len(a) for a in arrays])
     flat = np.ascontiguousarray(np.concatenate([np.asarray(a, dtype=np.uint64).reshape(-1, 2) for a in arrays] + [np.zeros((1, 2), np.uint64)]))
-    lib().wm_radix_sort_128x_batch(n, _p(flat, u64p), _p(off, i64p))
-    return [flat[off[i]: off[i + 1]].copy() for i in range(n)]
+    ms = C.c_float(0.0)
+    if timed:
+        lib().wm_radix_sort_128x_batch_timed(n, _p(flat, u64p), _p(off, i64p), C.byref(ms))
+    else:
+        lib().wm_radix_sort_128x_batch(n, _p(flat, u64p), _p(off, i64p))
+    out = [flat[off[i]: off[i + 1]].copy() for i in range(n)]
+    return (out, ms.value) if timed else out
 
 
 def chain_dp_batch(arrays, max_dist_x, min_dist_x, max_dist_y, bw, max_skip=25, max_iter=5000, min_cnt=3, min_sc=40, gap_scale=1.0):
